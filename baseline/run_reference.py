@@ -1,7 +1,7 @@
 """Times the UNMODIFIED reference's multiprocess CPU self-play path (TrainingLoop._generate_games,
 oinkoink/neural/training.py:99-133: game_pool worker processes x game threads + one InferenceServer process) on the host
-cores.  The reference package is imported from baseline/_ref (a git-ignored copy of /root/reference/oinkoink made by
-__graft_entry__.build(); it travels to the GPU box with the snapshot) with oracle/ref_shim standing in for the three
+cores.  The reference package is imported from baseline/_ref/oinkoink (a git-ignored copy of the unmodified package, put
+there by hand) with oracle/ref_shim standing in for the three
 uninstalled imports (anytree, matplotlib.pyplot, visdom).  Nothing of this package is on the path.  Prints one JSON line.
 Used by bench.py's cpu_baseline leg only (context next to the C port; see DESIGN.md section 5).
 usage: run_reference.py --procs P --threads T --games-per-proc N [--sims 800]"""
@@ -24,7 +24,7 @@ def main():
     a = ap.parse_args()
     ref = os.path.join(HERE, "_ref")
     if not os.path.isdir(os.path.join(ref, "oinkoink")):
-        print(json.dumps({"unavailable": "baseline/_ref/oinkoink is absent (build() copies it where /root/reference exists)"}))
+        print(json.dumps({"unavailable": "baseline/_ref/oinkoink is absent (copy the unmodified reference package there)"}))
         return
     sys.path.insert(0, os.path.join(ROOT, "oracle", "ref_shim"))
     sys.path.insert(0, ref)

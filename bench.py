@@ -30,9 +30,15 @@ A "step" = one such generation: fresh pool, empty memo, until `--games` games ha
           `traffic` = DRAM bytes per launch from the committed ncu capture of the same command and launch shape
           (profiles/r02_split_adapt_launches.csv; split engine, default workload), else null: no DRAM counter is read inside a run.
   cpu_baseline = the oracle port (oracle/selfplay_port.py) on the box's host cores, bounded sample (rank 0, N=1 only).
-  cpu_baseline_reference = the unmodified reference package (baseline/_ref, copied by build()) on the same cores: its
-          multiprocess game_pool + InferenceServer path, a bounded sample of whole games -- context for how conservative the port is.
+  cpu_baseline_reference = the unmodified reference package (baseline/_ref, a git-ignored copy put there by hand; reported
+          as unavailable without it) on the same cores: its multiprocess game_pool + InferenceServer path, a bounded sample of
+          whole games -- context for how conservative the port is.
 --impl reference: the CPU port alone, all host cores, same metric / config.
+--dump-outputs DIR: after the timed steps, DIR/<name>.npy (float64 / float32) holds what a caller received from them:
+  step_{positions,games,evals,memo_hits} = the counters of the last timed step (rank 0; they depend on where the stop lands,
+  so they vary slightly from run to run), and records_<field> = the position records of the timed end-to-end generation
+  (unless --no-e2e), sorted by game and ply; a seeded sample of rows keeps the whole dump under 64 MB.  The inputs are
+  seeded, so two builds run with the same arguments can be compared array by array.
 """
 import argparse
 import json
@@ -51,6 +57,7 @@ SIMS = 800
 STATE = os.path.join(ROOT, "tests", "golden", "example_net_state.npz")
 WORKLOAD = ("BASELINE.json configs[2]: 4096 concurrent self-play games per GPU, default NetConfig 32f/3r/4fc "
             "(example_net weights), 800 sims/move, AlphaZero noise alpha=0.3 frac=0.25, 6 sampled moves, 16-bit (fp16 operand / fp32 accumulate) tensor-core leaf eval")
+DUMP_BYTES = 63 << 20                                   # --dump-outputs: record columns; with the rest under 64 MB
 
 
 def peaks():
@@ -183,6 +190,24 @@ def digest_records(rec):
     return h.hexdigest()[:16]
 
 
+def dump_outputs(path, step, rec):
+    """--dump-outputs: the last timed step's counters and the end-to-end generation's records (or None) as .npy files"""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    out = {"step_" + k: np.array([step[k]], np.float64) for k in ("positions", "games", "evals", "memo_hits")}
+    if rec is not None:
+        rec = rec[np.lexsort((rec["ply"], rec["game_id"]))]          # the engine writes records in the order games finish
+        cols = {"records_" + f: rec[f].astype(np.float64) for f in ("c0", "c1", "game_id", "move", "ply", "n_moves", "result")}
+        cols.update({"records_" + f: rec[f].astype(np.float32) for f in ("policy", "result_value", "search_value")})
+        row_bytes = sum(a.nbytes for a in cols.values()) // max(1, len(rec))
+        if len(rec) * row_bytes > DUMP_BYTES:
+            keep = np.sort(np.random.default_rng(0).choice(len(rec), DUMP_BYTES // row_bytes, replace=False))
+            cols = {k: a[keep] for k, a in cols.items()}
+        out.update(cols)
+    for k, a in out.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+
+
 def ncu_traffic(path, kernel="k_sp_one"):
     """mean over the launches of `kernel` in an ncu --csv metrics file of dram__bytes_read.sum + dram__bytes_write.sum (bytes), or None"""
     import csv
@@ -215,12 +240,17 @@ def main():
     ap.add_argument("--no-ref-python", action="store_true", help="skip the unmodified-reference CPU sample (about 40 s)")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip generation_1200 / steady_state / engine A-B")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the timed steps to DIR/<name>.npy (see above)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs needs --impl ours")
         run_reference(args, rank)
         return
 
@@ -284,7 +314,7 @@ def main():
     value = positions / secs
 
     # end to end through the public API with host buffers: one whole generation, records back on the host
-    e2e = None
+    e2e = e2e_rec = None
     if not args.no_e2e:
         n_e2e = args.e2e_games * world
         start = (torch.zeros(args.e2e_games, dtype=torch.int64).pin_memory(),               # host-resident (pinned) inputs:
@@ -327,7 +357,10 @@ def main():
                "rank0_phase_seconds": {k: round(v, 4) for k, v in phases.items()} if world > 1 else None,
                "records_sha256_16": digest_records(rec) if world > 1 and rec is not None else None}
         pool2.engine.close()
+        e2e_rec = rec if args.dump_outputs else None
         del rec
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, r, e2e_rec)
 
     extras = {}
     if not args.no_extras:
