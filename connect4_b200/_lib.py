@@ -2,6 +2,7 @@
 compute entry point is called without a usable GPU, the call raises."""
 import ctypes as C
 import os
+import threading
 
 from . import _build
 
@@ -29,6 +30,9 @@ class RecordC(C.Structure):
 
 assert C.sizeof(RecordC) == 64
 
+# c4_eval_fn: the evaluator of a caller-served network (c4_net_create_external)
+EVAL_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p)
+
 # every symbol declared in include/c4b200.h : (restype, argtypes)
 SIGNATURES = {
     "c4_last_error": (C.c_char_p, []),
@@ -43,6 +47,7 @@ SIGNATURES = {
     "c4_board_from_planes": (C.c_int, [vp, vp, vp, vp, C.c_int64, vp]),
     "c4_board_evaluate_centre": (C.c_int, [vp, vp, vp, C.c_int64, vp]),
     "c4_net_create": (C.c_int, [C.c_int, vp, C.c_int64, C.POINTER(vp)]),
+    "c4_net_create_external": (C.c_int, [C.c_int, EVAL_FN, vp, C.POINTER(vp)]),
     "c4_net_destroy": (C.c_int, [vp]),
     "c4_net_forward": (C.c_int, [vp, vp, vp, C.c_int64, vp, vp, vp]),
     "c4_net_flops_per_position": (C.c_double, [vp]),
@@ -100,9 +105,22 @@ def load():
     return L
 
 
+_callback_error = threading.local()
+
+
+def set_callback_error(exc):
+    """remember the exception a Python evaluator raised inside a c4_eval_fn callback (which can only return non-zero);
+    the failing engine call re-raises it as the cause of its C4Error"""
+    _callback_error.exc = exc
+
+
 def check(rc):
     if rc != 0:
-        raise C4Error(load().c4_last_error().decode() or "libc4b200 error %d" % rc)
+        msg = load().c4_last_error().decode() or "libc4b200 error %d" % rc
+        cause, _callback_error.exc = getattr(_callback_error, "exc", None), None
+        if cause is None:
+            raise C4Error(msg)
+        raise C4Error("%s: %s: %s" % (msg, type(cause).__name__, cause)) from cause
 
 
 def require_gpu():

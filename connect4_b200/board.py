@@ -204,6 +204,10 @@ def expand(ips, board, plies):
         expand(ips, nb, plies - 1)
 
 
+# element types of c4_board_to_planes (include/c4b200.h)
+PLANE_DTYPES = {"uint8": 0, "float32": 1, "float16": 2, "bfloat16": 3}
+
+
 class BoardBatch():
     """n positions as two uint64 CUDA tensors (viewed through int64 storage); batched bitboard engine on the GPU."""
 
@@ -263,11 +267,13 @@ class BoardBatch():
         return BoardBatch(f0, f1)
 
     def to_planes(self, dtype="uint8"):
+        """Board.to_array of every position: [n, 3, 6, 7] in "uint8", "float32", "float16" or "bfloat16" """
         import torch
         from ._lib import ptr
-        td = torch.uint8 if dtype == "uint8" else torch.float32
+        code = PLANE_DTYPES.get(dtype, 1)                  # (any other name: float32)
+        td = (torch.uint8, torch.float32, torch.float16, torch.bfloat16)[code]
         out = torch.empty((self.n, 3, 6, 7), dtype=td, device="cuda")
-        self._call("c4_board_to_planes", ptr(self.c0), ptr(self.c1), ptr(out), 0 if dtype == "uint8" else 1, self.n)
+        self._call("c4_board_to_planes", ptr(self.c0), ptr(self.c1), ptr(out), code, self.n)
         return out
 
     @classmethod

@@ -1,5 +1,8 @@
 // c4_board.cu -- batched bitboard engine kernels + their C-ABI entry points (include/c4b200.h).
 // One thread per position, grid-stride, 64-bit coalesced loads; pure integer work, HBM-bound (16-32 B/position).
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
+
 #include "c4_common.cuh"
 
 static thread_local std::string g_err;
@@ -68,6 +71,9 @@ __global__ void k_fliplr(const u64 *__restrict__ c0, const u64 *__restrict__ c1,
 // TP positions in shared memory -- one thread per (position, channel, row) task writes that row's 7 values -- and then
 // streams the tile to global memory with 128-bit stores (a tile of TP positions is a multiple of 16 bytes).
 #define TP 64
+template <typename T> __device__ __forceinline__ T plane_value(unsigned v) { return (T)v; }
+template <> __device__ __forceinline__ __half plane_value<__half>(unsigned v) { return __uint2half_rn(v); }
+template <> __device__ __forceinline__ __nv_bfloat16 plane_value<__nv_bfloat16>(unsigned v) { return __uint2bfloat16_rn(v); }
 template <typename T>
 __global__ void __launch_bounds__(256) k_to_planes(const u64 *__restrict__ c0, const u64 *__restrict__ c1, T *__restrict__ planes,
                                                   int64_t n)
@@ -80,13 +86,13 @@ __global__ void __launch_bounds__(256) k_to_planes(const u64 *__restrict__ c0, c
             const u64 a = c0[p0 + p], b = c1[p0 + p];
             T *dst = tile + p * 126 + cr * 7;
             if (ch == 0) {
-                const T tm = (T)((c4_age(a, b) & 1) == 0);
+                const T tm = plane_value<T>((c4_age(a, b) & 1) == 0);
 #pragma unroll
                 for (int c = 0; c < 7; c++) dst[c] = tm;
             } else {
                 const u64 row = ((ch == 1 ? a : b) >> (5 - r));               // column c of this row at bit 7c
 #pragma unroll
-                for (int c = 0; c < 7; c++) dst[c] = (T)((row >> (7 * c)) & 1ULL);
+                for (int c = 0; c < 7; c++) dst[c] = plane_value<T>((unsigned)((row >> (7 * c)) & 1ULL));
             }
         }
         __syncthreads();
@@ -172,15 +178,20 @@ extern "C" int c4_board_to_planes(const uint64_t *c0, const uint64_t *c1, void *
                                   void *stream)
 {
     C4_REQUIRE(n >= 0 && (n == 0 || (c0 && c1 && planes)), "c4_board_to_planes: null pointer");
-    C4_REQUIRE(dtype == 0 || dtype == 1, "c4_board_to_planes: dtype must be 0 (uint8) or 1 (float32)");
+    C4_REQUIRE(dtype >= 0 && dtype <= 3, "c4_board_to_planes: dtype must be 0 (uint8), 1 (float32), 2 (float16) or 3 (bfloat16)");
     if (n == 0) return 0;
     C4_REQUIRE(((uintptr_t)planes & 15) == 0, "c4_board_to_planes: planes must be 16-byte aligned");
     const int64_t tiles = (n + TP - 1) / TP;
     const int blocks = (int)(tiles < 148 * 8 ? tiles : 148 * 8);
+    const cudaStream_t s = (cudaStream_t)stream;
     if (dtype == 0)
-        k_to_planes<uint8_t><<<blocks, 256, 0, (cudaStream_t)stream>>>((const u64 *)c0, (const u64 *)c1, (uint8_t *)planes, n);
+        k_to_planes<uint8_t><<<blocks, 256, 0, s>>>((const u64 *)c0, (const u64 *)c1, (uint8_t *)planes, n);
+    else if (dtype == 1)
+        k_to_planes<float><<<blocks, 256, 0, s>>>((const u64 *)c0, (const u64 *)c1, (float *)planes, n);
+    else if (dtype == 2)
+        k_to_planes<__half><<<blocks, 256, 0, s>>>((const u64 *)c0, (const u64 *)c1, (__half *)planes, n);
     else
-        k_to_planes<float><<<blocks, 256, 0, (cudaStream_t)stream>>>((const u64 *)c0, (const u64 *)c1, (float *)planes, n);
+        k_to_planes<__nv_bfloat16><<<blocks, 256, 0, s>>>((const u64 *)c0, (const u64 *)c1, (__nv_bfloat16 *)planes, n);
     LAUNCH_CHECK();
     return 0;
 }

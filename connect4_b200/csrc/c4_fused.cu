@@ -554,6 +554,7 @@ k_fused(const C4Dev dg, const unsigned char *__restrict__ image, int R, FzParams
 // can the fused engine run this network on a pool of this size at all?
 bool c4_fused_supported(const c4_net *net, int max_games)
 {
+    // (a network served by the caller, c4_net_create_external, has F = 0 and no images: it runs lock-step only)
     if (!net || (net->F != 32 && net->F != 64) || !net->use_tc || !net->image_tc) return false;
     int dev = 0, sms = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return false;

@@ -734,6 +734,8 @@ static int calibrate_range(c4_net *net, float *max_abs)
     return 0;
 }
 
+static unsigned long long next_net_uid = 1;   // c4_net::uid of the next network created
+
 extern "C" int c4_net_create(int device, const float *blob, int64_t n_floats, c4_net **out)
 {
     C4_REQUIRE(blob && out, "c4_net_create: null pointer");
@@ -751,9 +753,8 @@ extern "C" int c4_net_create(int device, const float *blob, int64_t n_floats, c4
     C4_REQUIRE(device >= 0 && device < ndev, "no such CUDA device (there is no CPU fallback)");
     C4_CUDA(cudaSetDevice(device));
 
-    static unsigned long long next_uid = 1;
     c4_net *net = new c4_net();
-    net->uid = next_uid++;
+    net->uid = next_net_uid++;
     net->device = device; net->F = F; net->R = R; net->n_fc = n_fc; net->fp16 = fp16;
     net->image = nullptr; net->image_tc = nullptr;
     net->scale_log2 = 0; net->calib_max = 0.f;
@@ -822,12 +823,34 @@ extern "C" int c4_net_create(int device, const float *blob, int64_t n_floats, c4
     return 0;
 }
 
+extern "C" int c4_net_create_external(int device, c4_eval_fn fn, void *user, c4_net **out)
+{
+    C4_REQUIRE(fn && out, "c4_net_create_external: null pointer");
+    int ndev = 0;
+    C4_CUDA(cudaGetDeviceCount(&ndev));
+    C4_REQUIRE(device >= 0 && device < ndev, "no such CUDA device (there is no CPU fallback)");
+    C4_CUDA(cudaSetDevice(device));
+    c4_net *net = new c4_net();
+    if (cudaMallocHost((void **)&net->ext_count, sizeof(int32_t)) != cudaSuccess) {
+        delete net;
+        c4_set_error("cudaMallocHost failed");
+        return -2;
+    }
+    net->uid = next_net_uid++;
+    net->device = device;
+    net->ext_fn = fn;
+    net->ext_user = user;
+    *out = net;
+    return 0;
+}
+
 extern "C" int c4_net_destroy(c4_net *net)
 {
     if (!net) return 0;
     cudaSetDevice(net->device);
     if (net->image) cudaFree(net->image);
     if (net->image_tc) cudaFree(net->image_tc);
+    if (net->ext_count) cudaFreeHost(net->ext_count);
     delete net;
     return 0;
 }
@@ -836,6 +859,7 @@ extern "C" double c4_net_flops_per_position(const c4_net *net) { return net ? ne
 extern "C" double c4_net_get(const c4_net *net, int key)
 {
     if (!net) return -1.0;
+    if (net->ext_fn) return 0.0;                                 // a caller-served network has none of these
     switch (key) {
     case 0: return net->F;
     case 1: return net->R;
@@ -849,6 +873,7 @@ extern "C" double c4_net_get(const c4_net *net, int key)
 unsigned long long c4_net_uid(const c4_net *net) { return net ? net->uid : 0ULL; }   // internal (not part of the C ABI)
 int c4_net_filters(const c4_net *net) { return net ? net->F : 0; }                  // internal
 int c4_net_device(const c4_net *net) { return net ? net->device : -1; }             // internal
+bool c4_net_external(const c4_net *net) { return net && net->ext_fn; }             // internal
 
 extern "C" int c4_net_forward(c4_net *net, const uint64_t *c0, const uint64_t *c1, int64_t n, const int32_t *count,
                               float *out, void *stream)
@@ -865,6 +890,22 @@ int c4_net_forward_ex(c4_net *net, const uint64_t *c0, const uint64_t *c1, int64
     if (n == 0) return 0;
     cudaStream_t s = (cudaStream_t)stream;
     C4_CUDA(cudaSetDevice(net->device));
+    if (net->ext_fn) {
+        // caller-served network: the host needs the leaf count to hand over the batch, hence one synchronise per call
+        if (count) {
+            C4_CUDA(cudaMemcpyAsync(net->ext_count, count, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+            C4_CUDA(cudaStreamSynchronize(s));
+            n = std::min<int64_t>(n, std::max(0, *net->ext_count));
+            if (n == 0) return 0;
+        }
+        const int rc = net->ext_fn(net->ext_user, c0, c1, n, out, stream);
+        if (rc) {
+            c4_set_error("the caller's evaluator failed (c4_eval_fn returned " + std::to_string(rc) + ")");
+            return -5;
+        }
+        C4_CUDA(cudaSetDevice(net->device));                    // (the callback may have switched devices)
+        return 0;
+    }
     if (net->use_tc) {
         int grid = (int)std::min<int64_t>(std::max(1, std::min(max_ctas, 148)), n);
         auto k = net->F == 32 ? (net->fp16 ? k_net_tc<OpFP16, 32> : k_net_tc<OpBF16, 32>)

@@ -466,6 +466,8 @@ struct c4_ctx {
     int budget_net;                     // terminal re-visits a game may play through per pass (NET / EXTERNAL)
     int last_pending;
     bool supplied;
+    bool search_failed;                 // the network call of the last c4_search_run failed: its games wait for answers
+                                        // that never came, so only a new c4_search_begin may run searches again
     bool pool_fresh;                    // bench pool initialised
     long long last_launches;            // kernels launched by the last c4_selfplay_stream call
     cudaGraphExec_t chunk_graph[2];     // 64 lock-step passes of the re-seeding / generation pool captured once (no per-launch
@@ -565,6 +567,7 @@ extern "C" int c4_ctx_create(int device, int32_t max_games, const c4_mcts_config
     ctx->pool_parity[0] = ctx->pool_parity[1] = 0;
     ctx->last_pending = 0;
     ctx->supplied = true;
+    ctx->search_failed = false;
     ctx->pool_fresh = false;
     ctx->pool_engine = 0;
     ctx->chunk_graph[0] = ctx->chunk_graph[1] = nullptr;
@@ -762,10 +765,22 @@ static int launch_advance(c4_ctx *ctx, int mode, int n_games, int budget, cudaSt
     return launch_advance_pool<SP>(ctx, mode, 0, n_games, 0, ctx->parity, budget, s);
 }
 
+// A failed network call (the caller's evaluator of an external net) leaves games waiting for answers that never came and
+// PENDING memo tags nobody will replace: the pool and the search batch must not be continued.  The next
+// c4_search_begin / c4_selfplay_run / c4_selfplay_stream starts from fresh slots and a new memo epoch (the abandoned tags
+// then read as misses).
+static int net_failed(c4_ctx *ctx, int rc)
+{
+    ctx->pool_fresh = false;
+    ctx->search_failed = true;
+    return rc;
+}
+
 static int run_net(c4_ctx *ctx, cudaStream_t s)
 {
-    return c4_net_forward(ctx->net, (const uint64_t *)ctx->d.leaf_c0, (const uint64_t *)ctx->d.leaf_c1, ctx->max_games,
-                          &ctx->d.ctr->leaf_count[0][ctx->parity], ctx->net_out, s);
+    const int rc = c4_net_forward(ctx->net, (const uint64_t *)ctx->d.leaf_c0, (const uint64_t *)ctx->d.leaf_c1,
+                                  ctx->max_games, &ctx->d.ctr->leaf_count[0][ctx->parity], ctx->net_out, s);
+    return rc ? net_failed(ctx, rc) : 0;
 }
 
 static inline void pool_range(const c4_ctx *ctx, int pool, int *g0, int *n)
@@ -792,6 +807,7 @@ extern "C" int c4_search_begin(c4_ctx *ctx, const uint64_t *c0, const uint64_t *
     ctx->n_search = n;
     ctx->last_pending = 0;
     ctx->supplied = true;
+    ctx->search_failed = false;
     return 0;
 }
 
@@ -842,8 +858,13 @@ static int read_counters(c4_ctx *ctx, C4Counters *host, cudaStream_t s)
 }
 
 // the two device-side failure words: a network answer that was not finite, and the fused engine's watchdog
-static int check_device_errors(const C4Counters &c)
+static int check_device_errors(const c4_ctx *ctx, const C4Counters &c)
 {
+    if (c.net_nonfinite && c4_net_external(ctx->net)) {
+        c4_set_error("the caller's evaluator returned a non-finite value or prior: oinkoink/neural/pytorch/model.py:258-263 "
+                     "asserts here");
+        return -3;
+    }
     if (c.net_nonfinite) {
         c4_set_error("the network produced a non-finite value or prior (fp16 operand overflow or NaN weights; try "
                      "operand_dtype='bf16'): oinkoink/neural/pytorch/model.py:258-263 asserts here");
@@ -875,6 +896,7 @@ extern "C" int c4_search_run(c4_ctx *ctx, int eval_kind, void *stream)
     C4_REQUIRE(ctx, "c4_search_run: null context");
     C4_REQUIRE(eval_kind == C4_EVAL_CENTRE || eval_kind == C4_EVAL_NET, "c4_search_run: eval_kind must be CENTRE or NET");
     C4_REQUIRE(eval_kind != C4_EVAL_NET || ctx->net, "c4_search_run: no network attached (c4_ctx_set_net)");
+    C4_REQUIRE(!ctx->search_failed, "c4_search_run: the network failed during the last search; start again with c4_search_begin");
     cudaStream_t s = (cudaStream_t)stream;
     C4_CUDA(cudaSetDevice(ctx->device));
     int rc;
@@ -889,7 +911,7 @@ extern "C" int c4_search_run(c4_ctx *ctx, int eval_kind, void *stream)
         // every search of the batch in ONE persistent launch (c4_fused.cu)
         if ((rc = persistent_run(ctx, ctx->n_search, false, 0ULL, 0.0, s))) return rc;
         if ((rc = read_counters(ctx, &c, s))) return rc;
-        if ((rc = check_device_errors(c))) return rc;
+        if ((rc = check_device_errors(ctx, c))) return rc;
         C4_REQUIRE((long long)c.n_done >= ctx->n_search, "c4_search_run: the fused engine left searches unfinished");
         return 0;
     }
@@ -900,7 +922,7 @@ extern "C" int c4_search_run(c4_ctx *ctx, int eval_kind, void *stream)
             if ((rc = run_net(ctx, s))) return rc;
         }
         if ((rc = read_counters(ctx, &c, s))) return rc;
-        if ((rc = check_device_errors(c))) return rc;
+        if ((rc = check_device_errors(ctx, c))) return rc;
         if ((long long)c.n_done >= ctx->n_search) break;
         C4_REQUIRE(it < (1 << 20), "c4_search_run: did not terminate");
     }
@@ -981,7 +1003,7 @@ static int selfplay_passes(c4_ctx *ctx, int eval_kind, int n_passes, cudaStream_
                 if (smp) { C4_CUDA(cudaEventRecordWithFlags(ctx->eva[2 * ns + 1], ps, ev_flags)); C4_CUDA(cudaEventRecordWithFlags(ctx->evs[2 * ns], ps, ev_flags)); }
                 if ((rc = c4_net_forward_ex(ctx->net, (const uint64_t *)(ctx->d.leaf_c0 + g0), (const uint64_t *)(ctx->d.leaf_c1 + g0),
                                             n, &ctx->d.ctr->leaf_count[p][ctx->pool_parity[p]], ctx->net_out + (size_t)g0 * 8, ps,
-                                            ctx->net_ctas))) return rc;
+                                            ctx->net_ctas))) return net_failed(ctx, rc);
                 if (smp) C4_CUDA(cudaEventRecordWithFlags(ctx->evs[2 * ns + 1], ps, ev_flags));
             }
         }
@@ -1001,12 +1023,13 @@ static int selfplay_passes(c4_ctx *ctx, int eval_kind, int n_passes, cudaStream_
 // graph captured the first time (and again whenever a launch parameter changes: the stop count follows the number of
 // live games in the drain of a generation, the kernel arguments hold the context's device pointers and RNG settings): the
 // launches then follow each other on the device without host work in between.  C4_NO_GRAPH=1 keeps the plain launches.
+// A network served by the caller is host code between the launches, so its passes are never captured.
 static int selfplay_chunk(c4_ctx *ctx, int eval_kind, cudaStream_t s, bool sampled = false)
 {
     static const bool no_graph = getenv("C4_NO_GRAPH") != nullptr;
     const bool two = ctx->n_pools == 2 && eval_kind == C4_EVAL_NET;
     int ns = 0;
-    if (no_graph || two || eval_kind != C4_EVAL_NET || ctx->parity != 0)
+    if (no_graph || two || eval_kind != C4_EVAL_NET || ctx->parity != 0 || c4_net_external(ctx->net))
         return selfplay_passes(ctx, eval_kind, 64, s, sampled ? 64 : 0, &ns, 0);
     const int gi = sampled ? 1 : 0;
     const int stop = pass_stop_count(ctx, ctx->max_games);
@@ -1072,14 +1095,14 @@ extern "C" int c4_selfplay_run(c4_ctx *ctx, int eval_kind, int64_t n_games, int6
         // all their slots are idle (c4_fused.cu)
         if ((rc = persistent_run(ctx, std::min<long long>(n_games, ctx->max_games), true, 0ULL, 0.0, s))) return rc;
         if ((rc = read_counters(ctx, &c, s))) return rc;
-        if ((rc = check_device_errors(c))) return rc;
+        if ((rc = check_device_errors(ctx, c))) return rc;
         C4_REQUIRE((long long)c.games_finished >= n_games, "c4_selfplay_run: the fused engine left games unfinished");
     } else {
         ctx->live_games = std::min<long long>(n_games, ctx->max_games);
         for (long long it = 0;; it++) {
             if ((rc = selfplay_chunk(ctx, eval_kind, s))) return rc;
             if ((rc = read_counters(ctx, &c, s))) return rc;
-            if ((rc = check_device_errors(c))) return rc;
+            if ((rc = check_device_errors(ctx, c))) return rc;
             ctx->live_games = std::max<long long>(1, std::min<long long>(n_games - (long long)c.games_finished, ctx->max_games));
             if ((long long)c.games_finished >= n_games) break;
             if (use_fused(ctx, eval_kind, ctx->live_games)) {
@@ -1096,7 +1119,7 @@ extern "C" int c4_selfplay_run(c4_ctx *ctx, int eval_kind, int64_t n_games, int6
                 } else if ((rc = launch_advance<true>(ctx, eval_kind, ctx->max_games, -1, s))) return rc;
                 if ((rc = persistent_run(ctx, ctx->live_games, true, 0ULL, 0.0, s))) return rc;
                 if ((rc = read_counters(ctx, &c, s))) return rc;
-                if ((rc = check_device_errors(c))) return rc;
+                if ((rc = check_device_errors(ctx, c))) return rc;
                 C4_REQUIRE((long long)c.games_finished >= n_games, "c4_selfplay_run: the fused engine left games unfinished");
                 break;
             }
@@ -1261,7 +1284,7 @@ extern "C" int c4_selfplay_stream(c4_ctx *ctx, int eval_kind, int reset, int64_t
     k_sum_stats<<<1, 256, 0, s>>>(d.stat_evals, d.stat_positions, d.stat_hits, ctx->max_games, ctx->stats_dev);
     C4_CUDA(cudaMemcpyAsync(ctx->pinned + 40, ctx->stats_dev, 3 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
     if ((rc = read_counters(ctx, &c, s))) return rc;
-    if ((rc = check_device_errors(c))) return rc;
+    if ((rc = check_device_errors(ctx, c))) return rc;
     after[0] = ctx->pinned[40]; after[1] = ctx->pinned[41]; after[2] = c.games_finished; after[3] = ctx->pinned[42];
     float ms = 0.f;
     C4_CUDA(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));

@@ -883,6 +883,7 @@ extern "C" int c4_split_adapt_next(int sms, int max_games, int n_net, unsigned l
 
 static bool c4_split_supported(const c4_net *net, int max_games)
 {
+    // (a network served by the caller, c4_net_create_external, has F = 0 and no images: it runs lock-step only)
     if (!net || (net->F != 32 && net->F != 64) || !net->use_tc || !net->image_tc) return false;
     if (getenv("C4_SP_DISABLE")) return false;                            // (tests of the other engines' auto policy)
     const int sms = sp_sms();

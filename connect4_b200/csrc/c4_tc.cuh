@@ -39,6 +39,9 @@ struct c4_net {
     double flops;
     int scale_log2;       // fp16 operands: the trunk runs at activations * 2^-scale_log2 (chosen by calibration at creation)
     float calib_max;      // largest |activation| (scaled units) the calibration positions produced
+    c4_eval_fn ext_fn;    // caller-served network (c4_net_create_external): F = R = 0, no images, no kernel of ours
+    void *ext_user;
+    int32_t *ext_count;   // pinned host copy of a device leaf count
 };
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }

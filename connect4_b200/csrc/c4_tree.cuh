@@ -9,6 +9,7 @@
 unsigned long long c4_net_uid(const c4_net *net);     // c4_net.cu (internal)
 int c4_net_filters(const c4_net *net);
 int c4_net_device(const c4_net *net);
+bool c4_net_external(const c4_net *net);              // served by the caller (c4_net_create_external)
 
 enum { ST_IDLE = 0, ST_READY = 1, ST_WAIT = 2, ST_DONE = 3, ST_NEWROOT = 4,
        ST_WAITMEMO = 7 };     // the leaf is being evaluated for ANOTHER game: re-probe the memo instead of asking again

@@ -4,6 +4,10 @@
   model([Board, ...]) -> (values ndarray (N,), priors ndarray (N,7))   float32   (model.py:269-282)
   anything else       -> TypeError                                               (model.py:176-178)
 
+Networks the library compiles (32 or 64 filters, 1..16 residual blocks) run on its CUDA tower (`backend == "cuda"`); any
+other geometry is served by a torch restatement of the reference's Net through `TorchModel` (`backend == "torch"`,
+neural/torch_model.py): the search and self-play stay on the device engine, the network is called once per pass.
+
 Training (model.py:199-240) is outside this path and raises NotImplementedError.  Checkpoints use the reference's
 format (`net_state_dict` / `optimiser_state_dict` / `scheduler_state_dict`, model.py:242-250).
 """
@@ -15,7 +19,7 @@ import numpy as np
 from .. import _lib
 from ..board import Board
 from .config import ModelConfig, NetConfig
-from .weights import fold_state_dict
+from .weights import fold_state_dict, net_shape
 
 
 def _init_state_dict(nc: NetConfig):
@@ -62,59 +66,30 @@ def _init_state_dict(nc: NetConfig):
     return {k: v.detach().clone() for k, v in Params().state_dict().items()}
 
 
-class ModelWrapper():
-    def __init__(self, config: Optional[ModelConfig] = None, file_name: Optional[str] = None, state_dict=None,
-                 device: Optional[int] = None, operand_dtype: str = "fp16", kernel: str = "auto"):
-        import torch
-        _lib.require_gpu()
-        self.config = config if config is not None else ModelConfig()
-        self._extra = {}
-        if state_dict is not None:
-            sd = state_dict
-        elif file_name is not None:
-            checkpoint = torch.load(file_name, map_location="cpu", weights_only=False)
-            sd = checkpoint['net_state_dict']
-            self._extra = {k: v for k, v in checkpoint.items() if k != 'net_state_dict'}
-        else:
-            sd = _init_state_dict(self.config.net_config)
-        self.state_dict = {k: (v if torch.is_tensor(v) else torch.as_tensor(np.asarray(v))) for k, v in sd.items()}
-        self.device = torch.device("cuda", torch.cuda.current_device() if device is None else device)
-        self.operand_dtype = operand_dtype
-        self.kernel = kernel
-        blob = fold_state_dict(self.state_dict, operand_dtype, kernel)
-        h = C.c_void_p()
-        _lib.check(_lib.load().c4_net_create(self.device.index, blob.ctypes.data_as(C.c_void_p), blob.size, C.byref(h)))
-        self.c4_net = h
-        self.n_parameters = sum(int(v.numel()) for k, v in self.state_dict.items()
-                                if "running_" not in k and "num_batches" not in k and not k.endswith((".w1", ".w2")))
-        print("Constructed NN with {} parameters".format(self.n_parameters))
+def compiled_geometry(filters: int, n_residuals: int, kernel: str = "auto") -> bool:
+    """True where c4_net_create accepts the network's shape (include/c4b200.h): the CUDA tower runs it.  `kernel` other than
+    "auto" asks for a particular CUDA kernel, so such a network always goes to c4_net_create (and fails there if it must)."""
+    return kernel != "auto" or (filters in (32, 64) and 1 <= n_residuals <= 16)
 
-    def __del__(self):
-        try:
-            if getattr(self, "c4_net", None):
-                _lib.load().c4_net_destroy(self.c4_net)
-                self.c4_net = None
-        except Exception:
-            pass
 
-    @property
-    def flops_per_position(self):
-        return float(_lib.load().c4_net_flops_per_position(self.c4_net))
+def flops_per_position(filters: int, n_residuals: int, n_fc: int) -> float:
+    """FLOPs (2*MAC, convs + linears) per position of a network of this shape (c4_net_flops_per_position)"""
+    F, R = filters, n_residuals
+    return 2.0 * (42.0 * 27 * F + 2.0 * R * 42 * 9 * F * F + 42.0 * F + n_fc * 42 * 42 + 42 + 42.0 * F * 2 + 84.0 * 7)
 
-    @property
-    def trunk_scale_log2(self):
-        """k of the power-of-two trunk scale 2^-k chosen at creation so that fp16 operands cannot overflow (0 for
-        networks in the usual activation range; see c4_net_get in include/c4b200.h)"""
-        return int(_lib.load().c4_net_get(self.c4_net, 3))
 
-    # ---- evaluator protocol
+class NetEvaluator():
+    """The reference's evaluator protocol and evaluation passes on top of a c4_net handle (`self.c4_net`, `self.device`):
+    shared by ModelWrapper and TorchModel, whatever serves the network."""
+
     def __call__(self, input_: Union[Board, List[Board]]):
         if isinstance(input_, Board):
             v, p = self._call_list([input_])
             return v.reshape(-1), p.reshape(-1)
         elif isinstance(input_, list):
             return self._call_list(input_)
-        raise TypeError('ModelWrapper called with {}. It accepts either a Board nor a list(Board)'.format(type(input_)))
+        raise TypeError('{} called with {}. It accepts either a Board nor a list(Board)'.format(type(self).__name__,
+                                                                                              type(input_)))
 
     def _call_list(self, board_list: List[Board]):
         c0 = np.array([int(b.color[0]) for b in board_list], np.uint64)
@@ -140,7 +115,7 @@ class ModelWrapper():
     # ---- evaluation pass over a labelled set (model.py:180-198,307-342; TrainingLoop._evaluate, training.py:156-171)
     def _eval_batches(self, data, batch_size, shuffle):
         """yields (value_out, prior_out, value_label, prior_label-or-None) CUDA tensors per mini-batch; the positions
-        go plane tensor -> bitboards (c4_board_from_planes) -> CUDA tower, nothing is evaluated on the host."""
+        go plane tensor -> bitboards (c4_board_from_planes) -> the network, nothing is evaluated on the host."""
         import torch
         from ..board import BoardBatch
         n = len(data)
@@ -173,6 +148,64 @@ class ModelWrapper():
             assert v.shape == yv.shape
             stats.update(v.cpu().numpy(), yv.cpu().numpy(), F.mse_loss(v, yv).item())
         return stats
+
+
+class ModelWrapper(NetEvaluator):
+    def __init__(self, config: Optional[ModelConfig] = None, file_name: Optional[str] = None, state_dict=None,
+                 device: Optional[int] = None, operand_dtype: str = "fp16", kernel: str = "auto"):
+        import torch
+        _lib.require_gpu()
+        self.backend = None
+        self.config = config if config is not None else ModelConfig()
+        self._extra = {}
+        if state_dict is not None:
+            sd = state_dict
+        elif file_name is not None:
+            checkpoint = torch.load(file_name, map_location="cpu", weights_only=False)
+            sd = checkpoint['net_state_dict']
+            self._extra = {k: v for k, v in checkpoint.items() if k != 'net_state_dict'}
+        else:
+            sd = _init_state_dict(self.config.net_config)
+        self.state_dict = {k: (v if torch.is_tensor(v) else torch.as_tensor(np.asarray(v))) for k, v in sd.items()}
+        self.device = torch.device("cuda", torch.cuda.current_device() if device is None else device)
+        self.operand_dtype = operand_dtype
+        self.kernel = kernel
+        F, R, _ = net_shape(self.state_dict)
+        if compiled_geometry(F, R, kernel):
+            blob = fold_state_dict(self.state_dict, operand_dtype, kernel)
+            h = C.c_void_p()
+            _lib.check(_lib.load().c4_net_create(self.device.index, blob.ctypes.data_as(C.c_void_p), blob.size, C.byref(h)))
+            self.c4_net = h
+            self.backend = "cuda"
+        else:
+            from .torch_model import TorchModel, TorchNet
+            dt = {"fp16": torch.float16, "bf16": torch.bfloat16}[operand_dtype]
+            self._served = TorchModel(TorchNet(self.state_dict, dt).to(self.device), self.device, dt)
+            self.c4_net = self._served.c4_net
+            self.backend = "torch"
+        self.n_parameters = sum(int(v.numel()) for k, v in self.state_dict.items()
+                                if "running_" not in k and "num_batches" not in k and not k.endswith((".w1", ".w2")))
+        print("Constructed NN with {} parameters".format(self.n_parameters))
+
+    def __del__(self):
+        try:
+            if self.backend == "cuda" and getattr(self, "c4_net", None):     # (a TorchModel owns its own handle)
+                _lib.load().c4_net_destroy(self.c4_net)
+                self.c4_net = None
+        except Exception:
+            pass
+
+    @property
+    def flops_per_position(self):
+        if self.backend == "cuda":
+            return float(_lib.load().c4_net_flops_per_position(self.c4_net))
+        return flops_per_position(*net_shape(self.state_dict))
+
+    @property
+    def trunk_scale_log2(self):
+        """k of the power-of-two trunk scale 2^-k chosen at creation so that fp16 operands cannot overflow (0 for
+        networks in the usual activation range; see c4_net_get in include/c4b200.h)"""
+        return int(_lib.load().c4_net_get(self.c4_net, 3))
 
     # ---- checkpoints (reference format)
     def save(self, folder_path: str):

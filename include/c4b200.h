@@ -52,7 +52,8 @@ int c4_board_has_win(const uint64_t *bb, uint8_t *out, int64_t n, void *stream);
 int c4_board_result(const uint64_t *c0, const uint64_t *c1, int8_t *result_out, int64_t n, void *stream);
 /* Board.create_fliplr / flip_color (oinkoink/board.py:115-145) */
 int c4_board_fliplr(const uint64_t *c0, const uint64_t *c1, uint64_t *f0, uint64_t *f1, int64_t n, void *stream);
-/* Board.to_array (oinkoink/board.py:147-154): planes [n][3][6][7], row 0 = top; dtype 0 = uint8, 1 = float32 */
+/* Board.to_array (oinkoink/board.py:147-154): planes [n][3][6][7], row 0 = top; dtype 0 = uint8, 1 = float32,
+ * 2 = float16, 3 = bfloat16 (the operand type of a caller-served network, see c4_net_create_external) */
 int c4_board_to_planes(const uint64_t *c0, const uint64_t *c1, void *planes, int dtype, int64_t n, void *stream);
 /* Board.from_pieces colour part (oinkoink/board.py:43-50): uint8 planes o[n][6][7], x[n][6][7] -> bitboards */
 int c4_board_from_planes(const uint8_t *o, const uint8_t *x, uint64_t *c0, uint64_t *c1, int64_t n, void *stream);
@@ -71,6 +72,22 @@ int c4_board_evaluate_centre(const uint64_t *c0, const uint64_t *c1, double *val
  *   policy head: wp[2][F], bp[2]; fc W[7][84], b[7].
  * Supported: F in {32, 64}. */
 int c4_net_create(int device, const float *blob, int64_t n_floats, c4_net **out);
+/* A network the CALLER serves (any geometry, any framework): the engine keeps the tree passes, the evaluation memo and
+ * its de-duplication, leaf compaction, Philox noise and the records, and hands each compacted leaf batch to `fn`.
+ *   fn(user, c0, c1, n, out, stream): c0/c1 (DEVICE, n >= 1 leaves) -> out[i] = {prior[0..6], value} (DEVICE, the rows
+ *   c4_net_forward writes).  It is called on the thread that made the engine call, between the tree pass that compacted
+ *   the leaves and the next pass; its work must be enqueued on `stream` (a cudaStream_t, NULL = default stream) or
+ *   finished before it returns.  A non-zero return fails the engine call ("the caller's evaluator failed"); the context
+ *   stays usable: the next c4_search_begin / c4_selfplay_run / c4_selfplay_stream(reset=1) starts clean.
+ * The result is an ordinary c4_net: c4_ctx_set_net attaches it (with a fresh memo key), c4_net_forward calls `fn`
+ * (after reading a device `count`, which synchronises the stream; n = 0 leaves make no call), c4_net_destroy frees it.
+ * c4_net_get and c4_net_flops_per_position return 0 for it.
+ * Engine policy: an external network always runs on the lock-step pass engine (the persistent split / fused engines
+ * cannot call back into the host in the middle of a launch; C4_ENGINE=split|fused is ignored for it), with one host
+ * synchronise per pass, and no pass is captured into a CUDA graph.  A non-finite answer fails the call like one of the
+ * built-in tower. */
+typedef int (*c4_eval_fn)(void *user, const uint64_t *c0, const uint64_t *c1, int64_t n, float *out, void *stream);
+int c4_net_create_external(int device, c4_eval_fn fn, void *user, c4_net **out);
 int c4_net_destroy(c4_net *net);
 /* out[i] = {prior[0..6], value} as 8 float32 (DEVICE, 32 B per position); `count` (DEVICE int32, may be NULL)
  * overrides n with a device-side position count <= n. 16-bit tensor-core tower (fp16 operands by default, bf16
