@@ -6,8 +6,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libc4b200.so")
-SOURCES = ["c4_board.cu", "c4_search.cu", "c4_net.cu", "c4_fused.cu", "c4_split.cu"]
-HEADERS = ["c4_common.cuh", "c4_tree.cuh", "c4_tc.cuh", "c4_fz.cuh", os.path.join("..", "..", "include", "c4b200.h")]
+SOURCES = ["c4_board.cu", "c4_search.cu", "c4_net.cu", "c4_layers.cu", "c4_fused.cu", "c4_split.cu"]
+HEADERS = ["c4_common.cuh", "c4_tree.cuh", "c4_tc.cuh", "c4_fz.cuh", "c4_layers.cuh", os.path.join("..", "..", "include", "c4b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-O2"]
 

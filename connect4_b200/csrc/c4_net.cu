@@ -27,6 +27,7 @@
 #include "c4_common.cuh"
 
 #include "c4_tc.cuh"
+#include "c4_layers.cuh"
 
 // One 3x3 convolution of one board as implicit GEMM: acc[t][j][.] (+)= sum over taps/channels.
 //   src: padded activation strip (row stride AS bytes), W: [F][9*CIN + 8] bf16 rows (stride WS bytes)
@@ -547,7 +548,7 @@ k_net_tc(const unsigned char *__restrict__ image, int R, const u64 *__restrict__
 
 // ------------------------------------------------------------------------------------------------ host side
 int c4_net_forward_ex(c4_net *net, const uint64_t *c0, const uint64_t *c1, int64_t n, const int32_t *count, float *out,
-                      void *stream, int max_ctas);
+                      void *stream, int max_ctas, const c4_ly_scratch *scratch);
 static uint16_t f2bf(float f)
 {
     uint32_t u;
@@ -563,6 +564,27 @@ static uint16_t f2h(float f)
     uint16_t u;
     memcpy(&u, &h, 2);
     return u;
+}
+
+uint16_t c4_f2op(float f, bool fp16) { return fp16 ? f2h(f) : f2bf(f); }
+
+// head parameters of the blob (from the value head's 1x1 conv on) -> the fp32 head block; the 1x1 conv weights go to vw [F]
+// and pw [2][F]
+void c4_pack_heads(const float *p, int F, float *hp, float *vw, float *pw)
+{
+    memcpy(vw, p, F * 4); p += F;
+    hp[HO_VB] = *p++;
+    for (int i = 0; i < 42; i++)
+        for (int j = 0; j < 42; j++) hp[HO_FCT + j * 42 + i] = p[i * 42 + j];
+    p += 42 * 42;
+    memcpy(hp + HO_FCB, p, 42 * 4); p += 42;
+    memcpy(hp + HO_FC1W, p, 42 * 4); p += 42;
+    hp[HO_FC1B] = *p++;
+    hp[HO_W1] = *p++; hp[HO_W2] = *p++;
+    memcpy(pw, p, F * 4); memcpy(pw + F, p + F, F * 4); p += 2 * F;
+    hp[HO_PB] = *p++; hp[HO_PB + 1] = *p++;
+    memcpy(hp + HO_POLW, p, 7 * 84 * 4); p += 7 * 84;
+    memcpy(hp + HO_POLB, p, 7 * 4);
 }
 
 // pack W[co][ci][ky][kx] (fp32) into [co][k = (ky*3+kx)*CINP + ci] 16-bit rows of (9*CINP + 8) elements
@@ -647,19 +669,7 @@ static int upload_images(c4_net *net, const float *blob)
         memcpy(bias + (1 + l) * F, p, F * 4);
         p += F;
     }
-    memcpy(hp + HO_VW, p, F * 4); p += F;
-    hp[HO_VB] = *p++;
-    for (int i = 0; i < 42; i++)
-        for (int j = 0; j < 42; j++) hp[HO_FCT + j * 42 + i] = p[i * 42 + j];
-    p += 42 * 42;
-    memcpy(hp + HO_FCB, p, 42 * 4); p += 42;
-    memcpy(hp + HO_FC1W, p, 42 * 4); p += 42;
-    hp[HO_FC1B] = *p++;
-    hp[HO_W1] = *p++; hp[HO_W2] = *p++;
-    memcpy(hp + HO_PW, p, F * 4); memcpy(hp + HO_PW + F, p + F, F * 4); p += 2 * F;
-    hp[HO_PB] = *p++; hp[HO_PB + 1] = *p++;
-    memcpy(hp + HO_POLW, p, 7 * 84 * 4); p += 7 * 84;
-    memcpy(hp + HO_POLB, p, 7 * 4); p += 7;
+    c4_pack_heads(p, F, hp, hp + HO_VW, hp + HO_PW);
     net->image_bytes = total;
     if (!net->image && cudaMalloc(&net->image, total) != cudaSuccess) { c4_set_error("cudaMalloc failed"); return -2; }
     C4_CUDA(cudaMemcpy(net->image, img.data(), total, cudaMemcpyHostToDevice));
@@ -692,7 +702,8 @@ static int upload_images(c4_net *net, const float *blob)
 }
 
 // Largest |activation| any trunk layer produces on a fixed set of 512 calibration positions (random stones of both colours,
-// 0..40 plies, deterministic), measured with the tcgen05 kernel itself.  Inf / NaN come back as a huge value.
+// 0..40 plies, deterministic), measured with the kernel that runs the network (tcgen05 tower or layered kernels).  Inf / NaN
+// come back as a huge value.
 static int calibrate_range(c4_net *net, float *max_abs)
 {
     const int n = 512;
@@ -721,12 +732,17 @@ static int calibrate_range(c4_net *net, float *max_abs)
     C4_CUDA(cudaMemcpy(d0, c0.data(), n * 8, cudaMemcpyHostToDevice));
     C4_CUDA(cudaMemcpy(d1, c1.data(), n * 8, cudaMemcpyHostToDevice));
     C4_CUDA(cudaMemset(mx, 0, 64));
-    const int tc_smem = net->F == 32 ? TcK<32>::total(net->R) : TcK<64>::total(net->R);
-    auto k = net->F == 32 ? k_net_tc<OpFP16, 32, true> : k_net_tc<OpFP16, 64, true>;
-    C4_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, tc_smem));
-    k<<<32, TC_THREADS, tc_smem>>>((const unsigned char *)net->image_tc, net->R, d0, d1, n, nullptr, out,
-                                   reinterpret_cast<long long *>(mx));
-    C4_CUDA(cudaGetLastError());
+    if (net->layers) {
+        const int rc = c4_ly_forward(net, (const uint64_t *)d0, (const uint64_t *)d1, n, nullptr, out, 0, 148, nullptr, mx);
+        if (rc) return rc;
+    } else {
+        const int tc_smem = net->F == 32 ? TcK<32>::total(net->R) : TcK<64>::total(net->R);
+        auto k = net->F == 32 ? k_net_tc<OpFP16, 32, true> : k_net_tc<OpFP16, 64, true>;
+        C4_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, tc_smem));
+        k<<<32, TC_THREADS, tc_smem>>>((const unsigned char *)net->image_tc, net->R, d0, d1, n, nullptr, out,
+                                       reinterpret_cast<long long *>(mx));
+        C4_CUDA(cudaGetLastError());
+    }
     unsigned bits = 0;
     C4_CUDA(cudaMemcpy(&bits, mx, 4, cudaMemcpyDeviceToHost));
     cudaFree(d0); cudaFree(d1); cudaFree(out); cudaFree(mx);
@@ -742,9 +758,16 @@ extern "C" int c4_net_create(int device, const float *blob, int64_t n_floats, c4
     C4_REQUIRE(n_floats >= 4 && (int)blob[0] == 0xC4B2, "c4_net_create: bad blob magic");
     const int F = (int)blob[1], R = (int)blob[2], n_fc = (int)blob[3] & 0xff;
     const bool fp16 = (((int)blob[3] >> 8) & 0xff) != 1;        // header[3] = n_fc | (operand dtype << 8) | (kernel << 16)
-    const int kernel_sel = ((int)blob[3] >> 16) & 0xff;         // 0 = auto (tcgen05 when filters == 32), 1 = mma.sync
-    C4_REQUIRE(F == 32 || F == 64, "c4_net_create: filters must be 32 or 64");
-    C4_REQUIRE(R >= 1 && R <= 16, "c4_net_create: n_residuals out of range");
+    const int kernel_sel = ((int)blob[3] >> 16) & 0xff;         // 0 = auto (tcgen05 when filters == 32), 1 = mma.sync,
+                                                                // 2 = layer by layer (c4_layers.cu)
+    if (kernel_sel == 2) {
+        C4_REQUIRE(F >= 16 && F <= 256 && F % 16 == 0,
+                   "c4_net_create: the layered kernels need filters a multiple of 16 in 16..256");
+        C4_REQUIRE(R >= 1 && R <= 40, "c4_net_create: the layered kernels need n_residuals in 1..40");
+    } else {
+        C4_REQUIRE(F == 32 || F == 64, "c4_net_create: filters must be 32 or 64");
+        C4_REQUIRE(R >= 1 && R <= 16, "c4_net_create: n_residuals out of range");
+    }
     const int64_t expect = 4 + (int64_t)F * 27 + F + (int64_t)2 * R * ((int64_t)F * F * 9 + F) + F + 1 + 42 * 42 + 42 +
                            42 + 1 + 2 + 2 * F + 2 + 7 * 84 + 7;
     C4_REQUIRE(n_floats == expect, "c4_net_create: blob size does not match its header");
@@ -757,12 +780,16 @@ extern "C" int c4_net_create(int device, const float *blob, int64_t n_floats, c4
     net->uid = next_net_uid++;
     net->device = device; net->F = F; net->R = R; net->n_fc = n_fc; net->fp16 = fp16;
     net->image = nullptr; net->image_tc = nullptr;
+    net->layers = kernel_sel == 2; net->ly = nullptr;
     net->scale_log2 = 0; net->calib_max = 0.f;
     net->flops = 2.0 * (42.0 * 27 * F + 2.0 * R * 42 * 9 * F * F + 42.0 * F + (double)n_fc * 42 * 42 + 42 + 42.0 * F * 2 +
                         84.0 * 7);
     const int tc_smem = (F == 32) ? TcK<32>::total(R) : TcK<64>::total(R);
-    net->use_tc = kernel_sel != 1 && tc_smem <= 227 * 1024;
-    if (net->use_tc) {
+    net->use_tc = kernel_sel != 1 && !net->layers && tc_smem <= 227 * 1024;
+    int rc = 0;
+    if (net->layers) {
+        if ((rc = c4_ly_setup(net))) { c4_net_destroy(net); return rc; }
+    } else if (net->use_tc) {
         if (F == 32) {
             C4_CUDA(cudaFuncSetAttribute(k_net_tc<OpFP16, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc_smem));
             C4_CUDA(cudaFuncSetAttribute(k_net_tc<OpBF16, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc_smem));
@@ -771,7 +798,9 @@ extern "C" int c4_net_create(int device, const float *blob, int64_t n_floats, c4
             C4_CUDA(cudaFuncSetAttribute(k_net_tc<OpBF16, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc_smem));
         }
     }
-    if (F == 32) {
+    if (net->layers) {
+        // (no mma.sync kernel: c4_ly_setup above)
+    } else if (F == 32) {
         // the mma.sync kernel for 32 filters keeps every layer's weights resident in shared memory (up to 4 residual blocks);
         // deeper 32-filter networks run on the tcgen05 kernel only, which streams the weights layer by layer
         const bool resident_ok = smem_resident<32, WARPS_A>(R) <= 227 * 1024;
@@ -799,12 +828,12 @@ extern "C" int c4_net_create(int device, const float *blob, int64_t n_floats, c4
     // k = 0, i.e. exactly the unscaled arithmetic.  What calibration cannot foresee is caught at run time: a non-finite
     // network answer never enters a tree and makes the engine call fail (c4_search.cu / c4_fused.cu).
     std::vector<float> sb;
-    int rc = 0, k = 0;
+    int k = 0;
     bool ok = false;
     for (int attempt = 0; attempt < 12 && !ok; attempt++) {
         if (!scaled_blob(blob, n_floats, F, R, k, fp16, sb)) { k += 12; continue; }     // a weight overflows fp16
-        if ((rc = upload_images(net, sb.data()))) { c4_net_destroy(net); return rc; }
-        if (!fp16 || !net->use_tc || getenv("C4_NET_NO_CALIBRATION")) { ok = true; break; }
+        if ((rc = net->layers ? c4_ly_upload(net, sb.data()) : upload_images(net, sb.data()))) { c4_net_destroy(net); return rc; }
+        if (!fp16 || !(net->use_tc || net->layers) || getenv("C4_NET_NO_CALIBRATION")) { ok = true; break; }
         float m = 0.f;
         if ((rc = calibrate_range(net, &m))) { c4_net_destroy(net); return rc; }
         net->calib_max = m;
@@ -851,6 +880,7 @@ extern "C" int c4_net_destroy(c4_net *net)
     if (net->image) cudaFree(net->image);
     if (net->image_tc) cudaFree(net->image_tc);
     if (net->ext_count) cudaFreeHost(net->ext_count);
+    c4_ly_destroy(net);
     delete net;
     return 0;
 }
@@ -867,6 +897,7 @@ extern "C" double c4_net_get(const c4_net *net, int key)
     case 3: return net->scale_log2;
     case 4: return net->use_tc ? 1.0 : 0.0;
     case 5: return net->calib_max;
+    case 6: return net->layers ? 2.0 : net->use_tc ? 1.0 : 0.0;
     default: return -1.0;
     }
 }
@@ -874,16 +905,18 @@ unsigned long long c4_net_uid(const c4_net *net) { return net ? net->uid : 0ULL;
 int c4_net_filters(const c4_net *net) { return net ? net->F : 0; }                  // internal
 int c4_net_device(const c4_net *net) { return net ? net->device : -1; }             // internal
 bool c4_net_external(const c4_net *net) { return net && net->ext_fn; }             // internal
+bool c4_net_layered(const c4_net *net) { return net && net->layers; }              // internal
 
 extern "C" int c4_net_forward(c4_net *net, const uint64_t *c0, const uint64_t *c1, int64_t n, const int32_t *count,
                               float *out, void *stream)
 {
-    return c4_net_forward_ex(net, c0, c1, n, count, out, stream, 148);
+    return c4_net_forward_ex(net, c0, c1, n, count, out, stream, 148, nullptr);
 }
 
-// internal: same, with a cap on the number of CTAs (the self-play engine leaves SMs to the concurrent tree pass)
+// internal: same, with a cap on the number of CTAs (the self-play engine leaves SMs to the concurrent tree pass) and, for
+// a layered network, the activation scratch of the caller (null: the network's own, c4_ly_forward)
 int c4_net_forward_ex(c4_net *net, const uint64_t *c0, const uint64_t *c1, int64_t n, const int32_t *count, float *out,
-                      void *stream, int max_ctas)
+                      void *stream, int max_ctas, const c4_ly_scratch *scratch)
 {
     C4_REQUIRE(net && (n == 0 || (c0 && c1 && out)), "c4_net_forward: null pointer");
     C4_REQUIRE(n >= 0 && n < (1LL << 31), "c4_net_forward: n out of range");
@@ -906,7 +939,9 @@ int c4_net_forward_ex(c4_net *net, const uint64_t *c0, const uint64_t *c1, int64
         C4_CUDA(cudaSetDevice(net->device));                    // (the callback may have switched devices)
         return 0;
     }
-    if (net->use_tc) {
+    if (net->layers) {
+        return c4_ly_forward(net, c0, c1, n, count, out, s, max_ctas, scratch, nullptr);
+    } else if (net->use_tc) {
         int grid = (int)std::min<int64_t>(std::max(1, std::min(max_ctas, 148)), n);
         auto k = net->F == 32 ? (net->fp16 ? k_net_tc<OpFP16, 32> : k_net_tc<OpBF16, 32>)
                               : (net->fp16 ? k_net_tc<OpFP16, 64> : k_net_tc<OpBF16, 64>);

@@ -34,6 +34,7 @@
 #include "c4_common.cuh"
 
 #include "c4_tree.cuh"
+#include "c4_layers.cuh"
 
 // c4_fused.cu: the persistent engine (one launch per generation); c4_search.cu keeps the lock-step pass engine
 bool c4_fused_eligible(const c4_net *net, int max_games, long long live_games);
@@ -479,6 +480,7 @@ struct c4_ctx {
     cudaEvent_t ev0, ev1;
     cudaEvent_t evs[2 * 64];            // sampled (start, stop) pairs around network launches
     cudaEvent_t eva[2 * 64];            // sampled (start, stop) pairs around tree-pass launches
+    c4_ly_scratch ly_scr[2];            // layered network: activations of the whole pool / half pool 0, and of half pool 1
 };
 #define N_SAMPLES 64
 
@@ -572,6 +574,7 @@ extern "C" int c4_ctx_create(int device, int32_t max_games, const c4_mcts_config
     ctx->pool_engine = 0;
     ctx->chunk_graph[0] = ctx->chunk_graph[1] = nullptr;
     memset(ctx->chunk_key, 0, sizeof(ctx->chunk_key));
+    memset(ctx->ly_scr, 0, sizeof(ctx->ly_scr));
     memset(&ctx->d, 0, sizeof(ctx->d));
     C4Dev &d = ctx->d;
     // a warp starts no further descent in a NET pass after this many SM cycles (bounds the tail of the pass; 0 = off)
@@ -637,6 +640,7 @@ extern "C" int c4_ctx_destroy(c4_ctx *ctx)
     cudaSetDevice(ctx->device);
     for (int i = 0; i < 2; i++) if (ctx->chunk_graph[i]) cudaGraphExecDestroy(ctx->chunk_graph[i]);
     for (void *p : ctx->allocs) cudaFree(p);
+    for (int i = 0; i < 2; i++) c4_ly_scratch_free(&ctx->ly_scr[i]);
     if (ctx->pinned) cudaFreeHost(ctx->pinned);
     if (ctx->ev0) {
         cudaEventDestroy(ctx->ev0); cudaEventDestroy(ctx->ev1); cudaEventDestroy(ctx->ev_fork);
@@ -709,8 +713,30 @@ extern "C" int c4_ctx_set_net(c4_ctx *ctx, c4_net *net)
     // Self-play with a 64-filter network is network-bound (124 us network vs 41 us tree per pass): there the two half
     // pools on two streams pay -- the tree pass of one half runs under the network launch of the other (+7-9 %,
     // tools/ramp64.py) -- while with the 32-filter network the game chains are the limit and one pool is faster.
-    if (!getenv("C4_POOLS")) ctx->n_pools = (c4_net_filters(net) == 64 && ctx->max_games >= 512) ? 2 : 1;
-    if (!getenv("C4_NET_CTAS")) ctx->net_ctas = (ctx->n_pools == 2 && c4_net_filters(net) == 64) ? 96 : 112;
+    // A layered network (c4_layers.cu) is network-bound at every width (~0.5 ms network vs 0.04 ms tree per pass at 64
+    // filters): two half pools, network launches at 112 CTAs, measured +9 % at 128 filters and +1 % at 64 against one
+    // captured pool (tools/external_net_bench.py with C4_POOLS=1 / 2, DESIGN.md 4.2.1).
+    const bool layered = c4_net_layered(net);
+    if (!getenv("C4_POOLS"))
+        ctx->n_pools = ((c4_net_filters(net) == 64 || layered) && ctx->max_games >= 512) ? 2 : 1;
+    if (!getenv("C4_NET_CTAS")) ctx->net_ctas = (ctx->n_pools == 2 && c4_net_filters(net) == 64 && !layered) ? 96 : 112;
+    if (layered) {
+        // its activations live in global memory: one scratch per concurrent network launch of this context (the whole
+        // pool or half pool 0, and half pool 1), allocated here so that no forward allocates or is captured doing so
+        const int half = (ctx->max_games + 1) / 2;
+        const int cap[2] = {std::min(ctx->max_games, 16384), ctx->n_pools == 2 ? std::min(ctx->max_games - half, 16384) : 0};
+        for (int i = 0; i < 2; i++) {
+            c4_ly_scratch &sc = ctx->ly_scr[i];
+            if (cap[i] == 0 || (sc.base && sc.F == c4_net_filters(net) && sc.cap >= cap[i])) continue;
+            C4_CUDA(cudaDeviceSynchronize());
+            c4_ly_scratch_free(&sc);
+            // captured passes hold the old scratch pointers
+            for (int g = 0; g < 2; g++)
+                if (ctx->chunk_graph[g]) { cudaGraphExecDestroy(ctx->chunk_graph[g]); ctx->chunk_graph[g] = nullptr; }
+            const int rc = c4_ly_scratch_alloc(c4_net_filters(net), cap[i], &sc);
+            if (rc) return rc;
+        }
+    }
     return 0;
 }
 
@@ -726,7 +752,7 @@ extern "C" int c4_ctx_set_rng(c4_ctx *ctx, int mode, uint64_t seed, double *nois
 }
 
 int c4_net_forward_ex(c4_net *net, const uint64_t *c0, const uint64_t *c1, int64_t n, const int32_t *count, float *out,
-                      void *stream, int max_ctas);
+                      void *stream, int max_ctas, const c4_ly_scratch *scratch);
 
 // a NET self-play pass ends once this many games of the pool wait (stop_frac of the live games; steps of 64 so that the
 // captured launch graphs survive the slow decline of the live games in the drain of a generation)
@@ -778,8 +804,9 @@ static int net_failed(c4_ctx *ctx, int rc)
 
 static int run_net(c4_ctx *ctx, cudaStream_t s)
 {
-    const int rc = c4_net_forward(ctx->net, (const uint64_t *)ctx->d.leaf_c0, (const uint64_t *)ctx->d.leaf_c1,
-                                  ctx->max_games, &ctx->d.ctr->leaf_count[0][ctx->parity], ctx->net_out, s);
+    const int rc = c4_net_forward_ex(ctx->net, (const uint64_t *)ctx->d.leaf_c0, (const uint64_t *)ctx->d.leaf_c1,
+                                     ctx->max_games, &ctx->d.ctr->leaf_count[0][ctx->parity], ctx->net_out, s, 148,
+                                     &ctx->ly_scr[0]);
     return rc ? net_failed(ctx, rc) : 0;
 }
 
@@ -1003,7 +1030,7 @@ static int selfplay_passes(c4_ctx *ctx, int eval_kind, int n_passes, cudaStream_
                 if (smp) { C4_CUDA(cudaEventRecordWithFlags(ctx->eva[2 * ns + 1], ps, ev_flags)); C4_CUDA(cudaEventRecordWithFlags(ctx->evs[2 * ns], ps, ev_flags)); }
                 if ((rc = c4_net_forward_ex(ctx->net, (const uint64_t *)(ctx->d.leaf_c0 + g0), (const uint64_t *)(ctx->d.leaf_c1 + g0),
                                             n, &ctx->d.ctr->leaf_count[p][ctx->pool_parity[p]], ctx->net_out + (size_t)g0 * 8, ps,
-                                            ctx->net_ctas))) return net_failed(ctx, rc);
+                                            ctx->net_ctas, &ctx->ly_scr[p]))) return net_failed(ctx, rc);
                 if (smp) C4_CUDA(cudaEventRecordWithFlags(ctx->evs[2 * ns + 1], ps, ev_flags));
             }
         }

@@ -33,6 +33,8 @@ struct c4_net {
     unsigned long long uid;  // unique per created network (the engine's evaluation memo is keyed on it)
     bool fp16;            // operand element type of the conv GEMMs (false: bf16)
     bool use_tc;          // tcgen05 kernel instead of the mma.sync kernels
+    bool layers;          // layer-by-layer kernels (c4_layers.cu): `image` holds their weights, `ly` their scratch
+    struct c4_ly_net *ly;
     void *image_tc;       // device: [L][WSTAGE_BYTES] weights + biases + head block (tcgen05 kernel)
     void *image;          // device: smem image (kernel A) / per-layer weight images (kernel B)
     size_t image_bytes;

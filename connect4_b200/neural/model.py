@@ -8,6 +8,11 @@ Networks the library compiles (32 or 64 filters, 1..16 residual blocks) run on i
 other geometry is served by a torch restatement of the reference's Net through `TorchModel` (`backend == "torch"`,
 neural/torch_model.py): the search and self-play stay on the device engine, the network is called once per pass.
 
+`kernel="layers"` runs any network with a multiple of 16 filters in 16..256 and 1..40 residual blocks on the library's
+layer-by-layer tcgen05 kernels instead (`backend == "cuda"`, one launch per conv layer, DESIGN.md 4.3).  The default
+route (`kernel="auto"`) does not use them yet: it still sends every geometry the fused tower cannot compile to TorchNet.
+Whether the auto route should switch is a separate decision, to be made on the measurements of DESIGN.md 4.0.
+
 Training (model.py:199-240) is outside this path and raises NotImplementedError.  Checkpoints use the reference's
 format (`net_state_dict` / `optimiser_state_dict` / `scheduler_state_dict`, model.py:242-250).
 """

@@ -37,14 +37,15 @@ def net_shape(sd):
 OPERAND_DTYPES = {"fp16": 0, "bf16": 1}
 
 
-KERNELS = {"auto": 0, "mma": 1}
+KERNELS = {"auto": 0, "mma": 1, "layers": 2}
 
 
 def fold_state_dict(sd, operand_dtype="fp16", kernel="auto"):
     """operand_dtype: element type of the tensor-core conv GEMMs (accumulation is always fp32). fp16 is the default
     because bf16 operands miss the 1e-2 parity bound on the reference's trained checkpoint (DESIGN.md)."""
     F, R, n_fc = net_shape(sd)
-    # kernel: "auto" = tcgen05/TMEM tower (32 and 64 filters); "mma" forces the mma.sync kernels
+    # kernel: "auto" = tcgen05/TMEM tower (32 and 64 filters); "mma" forces the mma.sync kernels; "layers" = the
+    # layer-by-layer tcgen05 kernels (filters a multiple of 16 in 16..256, 1..40 residual blocks)
     parts = [np.array([MAGIC, F, R, n_fc | (OPERAND_DTYPES[operand_dtype] << 8) | (KERNELS[kernel] << 16)], np.float64)]
     w, b = _fold(sd, "body.0.0.weight", None, "body.0.1")
     parts += [w.reshape(-1), b]

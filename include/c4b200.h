@@ -66,11 +66,17 @@ int c4_board_evaluate_centre(const uint64_t *c0, const uint64_t *c1, double *val
  * ------------------------------------------------------------------------------------------------------------ */
 /* `blob` (HOST, float32) is the BN-folded parameter image built by connect4_b200.neural.weights.fold_state_dict:
  *   [0] magic 0xC4B2 [1] filters F [2] n_residuals R [3] n_fc | (operand dtype << 8) | (kernel << 16)
- *       (dtype 0 = fp16, 1 = bf16; kernel 0 = auto: tcgen05 tower for F = 32, 1 = force the mma.sync kernels), then
+ *       (dtype 0 = fp16, 1 = bf16; kernel 0 = auto: tcgen05 tower for F = 32, 1 = force the mma.sync kernels,
+ *       2 = "layers": the layer-by-layer tcgen05 kernels, one launch per conv with the activations in global memory), then
  *   stem W[F][3][3][3] (co,ci,ky,kx), stem b[F]; per residual conv (2R of them): W[F][F][3][3], b[F];
  *   value head: wv[F], bv; fc W[42][42] (the n_fc affine layers pre-multiplied), fc b[42]; fc1 w[42], b; w1, w2;
  *   policy head: wp[2][F], bp[2]; fc W[7][84], b[7].
- * Supported: F in {32, 64}. */
+ * Supported: kernels 0 and 1: F in {32, 64}, 1 <= R <= 16; kernel 2: F a multiple of 16 in 16..256, 1 <= R <= 40, any
+ * n_fc.  A geometry outside these is refused before any device is looked for.
+ * Kernel 2 networks run on the lock-step pass engine only (the split / fused engines refuse them, also under C4_ENGINE):
+ * from 512 game slots on two half pools on two streams (measured faster than one pool), else one pool whose passes are
+ * captured into CUDA graphs like the tower's.  An engine context keeps their activations in scratch of its own, one per
+ * half pool (allocated by c4_ctx_set_net), so two contexts may share one network. */
 int c4_net_create(int device, const float *blob, int64_t n_floats, c4_net **out);
 /* A network the CALLER serves (any geometry, any framework): the engine keeps the tree passes, the evaluation memo and
  * its de-duplication, leaf compaction, Philox noise and the records, and hands each compacted leaf batch to `fn`.
@@ -91,7 +97,9 @@ int c4_net_create_external(int device, c4_eval_fn fn, void *user, c4_net **out);
 int c4_net_destroy(c4_net *net);
 /* out[i] = {prior[0..6], value} as 8 float32 (DEVICE, 32 B per position); `count` (DEVICE int32, may be NULL)
  * overrides n with a device-side position count <= n. 16-bit tensor-core tower (fp16 operands by default, bf16
- * selectable in the blob header), fp32 accumulation, fp32 residual stream. */
+ * selectable in the blob header), fp32 accumulation, fp32 residual stream.  A layered network (kernel 2) works through
+ * the batch in chunks in global scratch owned by the network: calls on different streams or threads are ordered one after
+ * the other on the device.  No host synchronise and no allocation on any built-in network. */
 int c4_net_forward(c4_net *net, const uint64_t *c0, const uint64_t *c1, int64_t n, const int32_t *count, float *out,
                    void *stream);
 /* FLOPs (2*MAC, convs + linears) per position of this network: the roofline numerator (SURVEY.md 8d) */
@@ -99,7 +107,8 @@ double c4_net_flops_per_position(const c4_net *net);
 /* Network read-out: key 0 = filters, 1 = residual blocks, 2 = operand type of the conv GEMMs (0 fp16, 1 bf16), 3 = k of
  * the power-of-two trunk scale 2^-k chosen at creation so that fp16 operands cannot overflow (0 for networks in the usual
  * range: exactly the unscaled arithmetic), 4 = 1 if the tcgen05 kernel runs it, 5 = largest |activation| (scaled units)
- * of the 512 calibration positions.  A non-finite network answer at run time never enters a search tree and makes the
+ * of the 512 calibration positions, 6 = kernel that runs it (0 mma.sync, 1 fused tcgen05 tower, 2 layered kernels; key 4
+ * is 0 for a layered network).  A non-finite network answer at run time never enters a search tree and makes the
  * engine call fail (the reference asserts: oinkoink/neural/pytorch/model.py:258-263,275-280). */
 double c4_net_get(const c4_net *net, int key);
 

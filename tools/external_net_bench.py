@@ -7,6 +7,8 @@ reset=True, cold_memo=True)`, positions/s = root moves played / device time), fo
                       (planes -> bitboards -> tower: the same numbers; the difference is the per-pass host round trip)
   native / torch 64f  the example_config shape (64 filters, 6 blocks, 6 fc; seeded init) on the tower and as a TorchNet
   torch 128f          128 filters, 6 blocks, 6 fc (seeded init) through ModelWrapper, which serves it with TorchNet
+  layers 64f / 128f   the 64f network above and the torch_128f state dict on the layer-by-layer kernels
+                      (ModelWrapper(kernel="layers"), lock-step engine; C4_POOLS=1 / 2 compares one pool with two half pools)
 For the lock-step runs the engine's samplers give the passes, the mean tree-pass time and the mean network time, which for
 an external network is the synchronise + the callback (c4_ctx_get keys 8-10).  One JSON line per case.
 
@@ -75,6 +77,10 @@ def main():
         ("torch_64f", lambda: TorchModel(TorchNet(sd64, torch.float16).to(dev), dev, torch.float16), None),
         ("torch_128f", lambda: ModelWrapper(ModelConfig(net_config=NetConfig(filters=128, n_fc_layers=6, n_residuals=6)),
                                             state_dict=net(128, 6, 6)), None),
+        ("layers_64f", lambda: ModelWrapper(ModelConfig(net_config=NetConfig(filters=64, n_fc_layers=6, n_residuals=6)),
+                                            state_dict=sd64, kernel="layers"), None),
+        ("layers_128f", lambda: ModelWrapper(ModelConfig(net_config=NetConfig(filters=128, n_fc_layers=6, n_residuals=6)),
+                                             state_dict=net(128, 6, 6), kernel="layers"), None),
     ]
     only = set(filter(None, args.only.split(",")))
     lines = []
@@ -94,7 +100,8 @@ def main():
                    positions=r["positions"], device_ms=round(r["device_ms"], 1),
                    positions_per_sec=round(r["positions"] / (r["device_ms"] / 1e3)),
                    evals=r["evals"], memo_hits=r["memo_hits"], passes=r["passes"],
-                   tree_ms=round(r["tree_ms"], 4), net_or_callback_ms=round(r["net_ms"], 4), **head)
+                   tree_ms=round(r["tree_ms"], 4), net_or_callback_ms=round(r["net_ms"], 4),
+                   pools=os.environ.get("C4_POOLS", "default"), **head)
         lines.append(out)
         print(json.dumps(out), flush=True)
         del pool, model
